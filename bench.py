@@ -30,6 +30,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: the bench leaves nothing in it
 
 import numpy as np  # noqa: E402
 
@@ -61,7 +62,12 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the secondary configs (2 and 5) reported under 'also'")
     ap.add_argument("--max-paths", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the film planes of the last timed step of the headline workload to DIR/<plane>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def peaks():
@@ -145,6 +151,29 @@ class ClockSampler:
         except OSError:
             pass
         return out
+
+
+DUMP_MAX_PIXELS = 1 << 20  # 10 float32 channels per pixel: at most 40 MiB per dump
+
+
+def dump_outputs(out_dir, store, w, h):
+    """The film a caller of the timed path receives, as float32 arrays with one row per pixel (row-major, y up):
+    color.npy and background.npy and normal.npy [n, 3], alpha.npy [n].  A frame of more than DUMP_MAX_PIXELS pixels is
+    sampled: pixels np.sort(np.random.default_rng(0).choice(w * h, DUMP_MAX_PIXELS, replace=False)), the same for every
+    run at that resolution, so that two builds can be compared output for output."""
+    import torch
+    npx = w * h
+    if npx > DUMP_MAX_PIXELS:
+        idx = np.sort(np.random.default_rng(0).choice(npx, DUMP_MAX_PIXELS, replace=False))
+    else:
+        idx = np.arange(npx)
+    sel = torch.from_numpy(idx).to(store.device)
+    os.makedirs(out_dir, exist_ok=True)
+    off = 0
+    for name, ch in (("color", 3), ("alpha", 1), ("background", 3), ("normal", 3)):
+        a = store[off * npx:(off + ch) * npx].view(npx, ch).index_select(0, sel).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if ch > 1 else a[:, 0])
+        off += ch
 
 
 def build_workload(cfgnum, scaling, world, res=None, samples=None):
@@ -272,8 +301,9 @@ class Bench:
         self.torch.distributed.all_reduce(t, op=self.torch.distributed.ReduceOp.SUM)
         return float(t.item())
 
-    def run_config(self, cfgnum, scaling, steps, warmup, breakdown=True, e2e=True, parity_tiles=6):
-        """One workload: resident-input `value`, per-kernel breakdown, e2e, N>1 parity.  Returns a dict (all ranks)."""
+    def run_config(self, cfgnum, scaling, steps, warmup, breakdown=True, e2e=True, parity_tiles=6, dump_dir=None):
+        """One workload: resident-input `value`, per-kernel breakdown, e2e, N>1 parity.  Returns a dict (all ranks).
+        With `dump_dir`, rank 0 writes the film of the last timed step there before anything else renders into it."""
         torch = self.torch
         from rayn_b200 import _lib as L
         from rayn_b200.dist import DistFilm, device_frame_desc
@@ -310,6 +340,8 @@ class Bench:
         wall_ms = (time.perf_counter() - t0) * 1e3
         ev_ms = e0.elapsed_time(e1)
         self.barrier()
+        if dump_dir is not None and rank == 0:
+            dump_outputs(dump_dir, film.store, w, h)
         st = r.stats()
         total_samples = self.allsum(float(st.paths))
         ms_per_step = self.allmax(max(ev_ms, lib_ms)) / steps
@@ -484,7 +516,7 @@ def main():
     b = Bench(args, rank, world, local_rank)
 
     clocks = ClockSampler(local_rank) if rank == 0 else None  # started before warm-up (nvidia-smi needs ~0.3 s to emit its first line)
-    main_res = b.run_config(args.config, args.scaling, args.steps, args.warmup, breakdown=True, e2e=not args.no_e2e)
+    main_res = b.run_config(args.config, args.scaling, args.steps, args.warmup, breakdown=True, e2e=not args.no_e2e, dump_dir=args.dump_outputs)
     clock_info = clocks.stop() if clocks else None
     cpu_ctx = b._cpu_ctx
 

@@ -6,8 +6,6 @@ import re
 import subprocess
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "rayn_b200.h")
 
@@ -71,15 +69,18 @@ def test_struct_layouts_match_the_c_compiler(tmp_path):
 
 
 def test_create_fails_loudly_without_a_gpu():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from rayn_b200 import _lib as L
-    from rayn_b200.film import Renderer
-    with pytest.raises(L.RaynError) as e:
-        Renderer(0)
-    assert e.value.code == L.RAYN_ERR_NO_DEVICE
-    assert "no CPU fallback" in str(e.value)
+    """In a process that sees no device (CUDA_VISIBLE_DEVICES empty), so that it holds on a machine with a GPU too."""
+    code = ("import sys; sys.path.insert(0, %r)\n"
+            "from rayn_b200 import _lib as L\n"
+            "from rayn_b200.film import Renderer\n"
+            "try:\n"
+            "    Renderer(0)\n"
+            "except L.RaynError as e:\n"
+            "    assert e.code == L.RAYN_ERR_NO_DEVICE, e.code\n"
+            "    assert 'no CPU fallback' in str(e), str(e)\n"
+            "    print('raised')\n" % ROOT)
+    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True)
+    assert r.returncode == 0 and r.stdout.strip() == "raised", r.stdout + r.stderr
 
 
 def test_product_never_touches_the_oracle():

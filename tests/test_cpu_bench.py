@@ -106,6 +106,33 @@ def test_clock_log_parsing(tmp_path):
     assert out["reasons"] == ["hw_thermal_slowdown", "sw_power_cap"]
 
 
+def test_dump_outputs_writes_every_film_plane_per_pixel(tmp_path, monkeypatch):
+    """--dump-outputs: the film store (color | alpha | background | normal planes) as float32 arrays with one row per pixel;
+    frames above DUMP_MAX_PIXELS are a seeded pixel sample, the same on every run, and the headline dump stays under 64 MiB."""
+    import numpy as np
+    import torch
+    b = _bench()
+    assert b.DUMP_MAX_PIXELS * 10 * 4 <= 64 << 20
+    w, h = 40, 30
+    npx = w * h
+    store = torch.arange(10 * npx, dtype=torch.float32)
+    s = store.numpy()
+    want = {"color": s[:3 * npx].reshape(npx, 3), "alpha": s[3 * npx:4 * npx], "background": s[4 * npx:7 * npx].reshape(npx, 3),
+            "normal": s[7 * npx:].reshape(npx, 3)}
+    b.dump_outputs(str(tmp_path / "full"), store, w, h)
+    assert sorted(os.listdir(tmp_path / "full")) == sorted(f"{k}.npy" for k in want)
+    for k, v in want.items():
+        got = np.load(tmp_path / "full" / f"{k}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, v), k
+    monkeypatch.setattr(b, "DUMP_MAX_PIXELS", 100)
+    b.dump_outputs(str(tmp_path / "a"), store, w, h)
+    b.dump_outputs(str(tmp_path / "b"), store, w, h)
+    idx = np.sort(np.random.default_rng(0).choice(npx, 100, replace=False))
+    for k, v in want.items():
+        a = np.load(tmp_path / "a" / f"{k}.npy")
+        assert np.array_equal(a, v[idx]) and np.array_equal(a, np.load(tmp_path / "b" / f"{k}.npy")), k
+
+
 def test_committed_traffic_profile_belongs_to_this_kernel_build():
     """bench.py reports `roofline.traffic` only from an ncu capture of THIS kernel build: profiles/r02_traffic.json is keyed by the
     hash of the kernel sources.  A kernel edit without a new capture must be noticed (the line then says traffic: null)."""
