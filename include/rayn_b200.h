@@ -32,14 +32,19 @@ extern "C" {
 
 #define RAYN_B200_ABI_VERSION 2
 
-/* ---- limits (fixed so the scene fits a kernel-parameter block) -------------------
- * CONTRACT CHANGE vs the reference: its stores are unbounded `Vec<Box<dyn ..>>` (src/hitable.rs:143,
- * src/material.rs:58, src/world.rs:7-13).  Here the whole scene rides in the 4 KB kernel-parameter constant bank
- * (warp-uniform operands then cost no load), which caps the counts; setup.rs needs 7 / 4 / 5.  upload_scene returns
- * RAYN_ERR_INVALID_ARG beyond these.                                                                              */
-#define RAYN_MAX_HITABLES 16
-#define RAYN_MAX_MATERIALS 16
-#define RAYN_MAX_LIGHTS 16
+/* ---- limits -----------------------------------------------------------------------
+ * The reference's stores are unbounded `Vec<Box<dyn ..>>` (src/hitable.rs:143, src/material.rs:58, src/world.rs:7-13).
+ * A scene of at most 16 hitables, 16 materials and 16 lights rides in the kernel-parameter constant bank (warp-uniform
+ * operands then cost no load; setup.rs needs 7 / 4 / 5); a larger one is uploaded once into tables in device memory that
+ * the context owns.  Both render the same film.  upload_scene returns RAYN_ERR_INVALID_ARG, naming the limit, beyond:
+ *   RAYN_MAX_HITABLES / RAYN_MAX_MATERIALS: the per-tile bin tables hold one row entry per hitable;
+ *   RAYN_MAX_LIGHTS: CONTRACT CHANGE vs the reference - the shading kernels exchange a packet's light choices one byte each;
+ *   RAYN_MAX_SDF_HITABLES: CONTRACT CHANGE vs the reference - every SDF hitable costs its own march, normals and shadow
+ *     kernel per depth and its own shadow-segment queue (pass memory per path grows with the SDF count).              */
+#define RAYN_MAX_HITABLES 1024
+#define RAYN_MAX_MATERIALS 1024
+#define RAYN_MAX_LIGHTS 256
+#define RAYN_MAX_SDF_HITABLES 16
 #define RAYN_FIS_TABLE_SIZE 512 /* FILTER_TABLE_SIZE, src/filter.rs:187 */
 
 /* ---- status codes ---------------------------------------------------------------- */
@@ -226,6 +231,8 @@ typedef struct RaynConfig {
 #define RAYN_FLAG_NO_DIV3 32     /* never select the three-operation sphere-fold division (see rayn_b200_debug_sdf_variant) */
 #define RAYN_FLAG_NO_GRAPH 16    /* launch every kernel directly; by default small single-pass frames (launch bound) are
                                     captured once into a CUDA graph and replayed with one launch                */
+#define RAYN_FLAG_SCENE_TABLES 4 /* upload every scene into device-memory tables, also one that fits the parameter block
+                                    (test and measurement hook: the film is the same either way)                  */
 
 #define RAYN_STAT_KERNELS 12
 typedef struct RaynStats {

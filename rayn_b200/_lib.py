@@ -17,9 +17,10 @@ LIB_NAME = os.environ.get("RAYN_B200_LIB", LIB_NAME)  # tuning experiments: an e
 LIB_PATH = os.path.join(_HERE, "_build", LIB_NAME)
 HOSTLIB_PATH = os.path.join(_HERE, "_build", "librayn_hostinputs.so")
 
-RAYN_MAX_HITABLES = 16
-RAYN_MAX_MATERIALS = 16
-RAYN_MAX_LIGHTS = 16
+RAYN_MAX_HITABLES = 1024
+RAYN_MAX_MATERIALS = 1024
+RAYN_MAX_LIGHTS = 256
+RAYN_MAX_SDF_HITABLES = 16
 RAYN_FIS_TABLE_SIZE = 512
 
 RAYN_OK = 0
@@ -39,6 +40,7 @@ MEM_HOST, MEM_DEVICE = 0, 1
 POST_COLOR_PLUS_BACKGROUND, POST_COLOR_ALPHA, POST_COLOR_ONLY, POST_BACKGROUND, POST_WORLD_NORMAL, POST_ALPHA = range(6)
 POST_BYTES = (3, 4, 3, 3, 3, 1)
 FLAG_TIMING, FLAG_SIMPLE_MARCH, FLAG_NO_GRAPH, FLAG_NO_DIV3, FLAG_NO_FOLD_ALL = 1, 2, 16, 32, 64
+FLAG_SCENE_TABLES = 4
 STAT_KERNELS = 12
 KERNEL_NAMES = ["raygen", "extend", "bin", "shade_pre", "shadow", "shade_post", "compact", "resolve", "misc", "normals", "extend_spheres", "gather"]
 

@@ -10,6 +10,7 @@
 
 #include <algorithm>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "rt_kernels.cuh"
@@ -60,21 +61,34 @@ struct RaynContext {
   cudaStream_t stream = nullptr;
   std::string err;
   bool has_scene = false;
-  DevScene scene;
+  DevScene scene;  // every field of the uploaded scene; the arrays only when it takes the inline path (!tables)
+  // large-scene path (more than SCENE_INLINE_MAX hitables, materials or lights, or RAYN_FLAG_SCENE_TABLES): the kernels take
+  // tscene, whose tables live in d_tables.  scene_gen counts uploads, so that a graph captured for other table contents
+  // is never replayed (the tables are rewritten in place; their pointers do not change).
+  bool tables = false;
+  TableScene tscene;
+  unsigned char* d_tables = nullptr;
+  size_t cap_tables = 0;
+  uint64_t scene_gen = 0;
+  std::vector<RaynHitable> h_hit;  // host copies of the uploaded descriptors (launch decisions)
+  std::vector<RaynMaterial> h_mat;
   int64_t cap_paths = 0;  // requested paths per pass
   // pass buffers
   int64_t alloc_paths = 0, alloc_q = 0, alloc_seg = 0;
   int alloc_lc_ns = 0;
   int alloc_tiles = 0;
   int64_t alloc_segcnt = 0;  // ints in PassBufs::seg_cnt
+  int64_t alloc_bins = 0;    // ints in PassBufs::bin_start
   size_t pass_bytes = 0;
   PassBufs pb;
   int* d_tile_ids = nullptr;
   int* d_batch_prefix = nullptr;  // [alloc_tiles + 1]
   int* d_work_ctr = nullptr;      // [WC_TOTAL] global work counters of the persistent kernels
   int n_sm = 148;
-  int occ_ext[SDFV_COUNT], occ_shd[SDFV_COUNT], occ_nrm[SDFV_COUNT];
-  int occ_pre = 8, occ_post = 8, occ_sph = 8;  // resident CTAs per SM of the work-list kernels
+  struct Occ {  // resident CTAs per SM of the persistent and work-list kernels, per scene type ([0] DevScene, [1] TableScene)
+    int ext[SDFV_COUNT], shd[SDFV_COUNT], nrm[SDFV_COUNT];
+    int pre = 8, post = 8, sph = 8;
+  } occ[2];
   int sdf_var[RAYN_MAX_HITABLES];  // march-kernel variant of every SDF hitable of the uploaded scene (rt_sdf2.cuh::sdf_variant)
   struct Div3Check { float min_r2, fixed_r2; bool ok; };
   std::vector<Div3Check> div3_cache;  // exhaustive fastdiv2_3 checks already run on this device
@@ -167,21 +181,25 @@ static void free_pass(RaynContext* c) {
   c->alloc_lc_ns = 0;
   c->alloc_tiles = 0;
   c->alloc_segcnt = 0;
+  c->alloc_bins = 0;
   c->pass_bytes = 0;
 }
 
-// bytes of pass state per path (what ensure_pass allocates), used to size passes against free device memory
-static size_t pass_bytes_per_path(int R, int QS, int seg_per_path, int lc_ns) {
+// bytes of pass state per path (what ensure_pass allocates), used to size passes against free device memory; the per-tile
+// tables (bin starts and segment counts, maxk + 1 and maxk ints per row) are spread over the tile's R paths
+static size_t pass_bytes_per_path(int R, int QS, int seg_per_path, int lc_ns, int maxk) {
+  const double tile_ints = (double)(maxk + 1) + (double)((QS + SEG_SLOTS - 1) / SEG_SLOTS) * maxk;
   return 6 * sizeof(float4) + 2 * sizeof(uint32_t) + 2 * sizeof(int) + (size_t)(((double)QS / R) * sizeof(int) + 1) + (size_t)lc_ns * sizeof(float4) +
-         (lc_ns > 4 ? 8 * sizeof(float) : 0) + (size_t)seg_per_path * 2 * sizeof(float4);
+         (lc_ns > 4 ? 8 * sizeof(float) : 0) + (size_t)seg_per_path * 2 * sizeof(float4) + (size_t)(tile_ints * sizeof(int) / R + 1);
 }
 
-static int32_t ensure_pass(RaynContext* ctx, int n_tiles, int R, int QS, int seg_per_path_total, int n_sdf, int lc_ns) {
+static int32_t ensure_pass(RaynContext* ctx, int n_tiles, int R, int QS, int seg_per_path_total, int n_sdf, int lc_ns, int maxk) {
   const int64_t need_paths = (int64_t)n_tiles * R, need_q = (int64_t)n_tiles * QS;
   const int64_t need_seg = need_paths * seg_per_path_total;  // all SDF queues together
-  const int64_t need_segcnt = (int64_t)n_tiles * ((QS + SEG_SLOTS - 1) / SEG_SLOTS) * RAYN_MAX_HITABLES;
+  const int64_t need_segcnt = (int64_t)n_tiles * ((QS + SEG_SLOTS - 1) / SEG_SLOTS) * maxk;
+  const int64_t need_bins = (int64_t)n_tiles * (maxk + 1);
   if (need_paths <= ctx->alloc_paths && need_q <= ctx->alloc_q && n_tiles <= ctx->alloc_tiles && need_seg <= ctx->alloc_seg && lc_ns <= ctx->alloc_lc_ns &&
-      need_segcnt <= ctx->alloc_segcnt)
+      need_segcnt <= ctx->alloc_segcnt && need_bins <= ctx->alloc_bins)
     return RAYN_OK;
   free_pass(ctx);
   PassBufs& p = ctx->pb;
@@ -207,11 +225,12 @@ static int32_t ensure_pass(RaynContext* ctx, int n_tiles, int R, int QS, int seg
   PASS_ALLOC(p.q_shade, need_q * sizeof(int));
   PASS_ALLOC(p.n_live, n_tiles * sizeof(int));
   PASS_ALLOC(p.n_slots, n_tiles * sizeof(int));
-  PASS_ALLOC(p.bin_start, (size_t)n_tiles * (RAYN_MAX_HITABLES + 1) * sizeof(int));
+  PASS_ALLOC(p.bin_start, (size_t)need_bins * sizeof(int));
+  ctx->alloc_bins = need_bins;
   PASS_ALLOC(ctx->d_tile_ids, n_tiles * sizeof(int));
   PASS_ALLOC(ctx->d_batch_prefix, ((size_t)n_tiles + 1) * sizeof(int));
   PASS_ALLOC(p.seg_cnt, need_segcnt * sizeof(int));
-  PASS_ALLOC(p.slot_prefix, (size_t)(1 + RAYN_MAX_HITABLES) * ((size_t)n_tiles + 1) * sizeof(int));
+  PASS_ALLOC(p.slot_prefix, (size_t)(1 + RAYN_MAX_SDF_HITABLES) * ((size_t)n_tiles + 1) * sizeof(int));
   p.prefix_stride = n_tiles + 1;
   ctx->alloc_segcnt = need_segcnt;
   PASS_ALLOC(p.nrm, need_paths * sizeof(float4));
@@ -286,6 +305,20 @@ struct DevTmp {
     default: { constexpr int V = SDFV_BOX_GENERIC; STMT; } break;                     \
   }
 
+template <class S>
+static cudaError_t query_occupancy(RaynContext::Occ& o) {
+  cudaError_t e = cudaSuccess;
+  for (int v = 0; v < SDFV_COUNT && e == cudaSuccess; ++v) {
+    DISPATCH_SDFV(v, e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.ext[v], k_extend_march<V, S>, EXT_T, 0);
+                  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.shd[v], k_shadow<V, S>, SHD_T, 0);
+                  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.nrm[v], k_normals<V, S>, SLOT_BLOCK, 0));
+  }
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.pre, k_shade_pre<S>, SLOT_BLOCK, 0);
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.post, k_shade_post<S>, SLOT_BLOCK, 0);
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.sph, k_extend_spheres<S>, EXT_BATCH, 0);
+  return e;
+}
+
 static void tile_grid_of(int W, int H, int tw, int th, int* ntx, int* nty) {
   *ntx = (W + W % tw) / tw;  // film.rs:399-404
   *nty = (H + H % th) / th;
@@ -344,14 +377,17 @@ int32_t rayn_b200_create(const RaynConfig* cfg, RaynContext** out_ctx) {
   if (e == cudaSuccess) e = cudaEventCreate(&ctx->ev0);
   if (e == cudaSuccess) e = cudaEventCreate(&ctx->ev1);
   // persistent kernels: exactly as many CTAs as can be resident (one wave), so every CTA pulls work until the pass is drained
+  // (the inline scene's kernels are instantiated here first, in this order: ptxas output depends on the module's entry order)
+  RaynContext::Occ& o = ctx->occ[0];
   for (int v = 0; v < SDFV_COUNT && e == cudaSuccess; ++v) {
-    DISPATCH_SDFV(v, e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->occ_ext[v], k_extend_march<V>, EXT_T, 0);
-                  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->occ_shd[v], k_shadow<V>, SHD_T, 0);
-                  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->occ_nrm[v], k_normals<V>, SLOT_BLOCK, 0));
+    DISPATCH_SDFV(v, e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.ext[v], k_extend_march<V, DevScene>, EXT_T, 0);
+                  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.shd[v], k_shadow<V, DevScene>, SHD_T, 0);
+                  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.nrm[v], k_normals<V, DevScene>, SLOT_BLOCK, 0));
   }
-  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->occ_pre, k_shade_pre, SLOT_BLOCK, 0);
-  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->occ_post, k_shade_post, SLOT_BLOCK, 0);
-  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->occ_sph, k_extend_spheres, EXT_BATCH, 0);
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.pre, k_shade_pre<DevScene>, SLOT_BLOCK, 0);
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.post, k_shade_post<DevScene>, SLOT_BLOCK, 0);
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.sph, k_extend_spheres<DevScene>, EXT_BATCH, 0);
+  if (e == cudaSuccess) e = query_occupancy<TableScene>(ctx->occ[1]);
   if (e != cudaSuccess) {
     cudaGetLastError();
     fail(nullptr, RAYN_ERR_CUDA, "context setup: %s", cudaGetErrorString(e));
@@ -389,6 +425,7 @@ void rayn_b200_destroy(RaynContext* ctx) {
   cudaFree(ctx->d_pack_ids);
   cudaFree(ctx->d_post);
   cudaFree(ctx->d_s1), cudaFree(ctx->d_s2), cudaFree(ctx->d_scr), cudaFree(ctx->d_fis), cudaFree(ctx->d_planes);
+  cudaFree(ctx->d_tables);
   for (auto& t : ctx->timed) cudaEventDestroy(t.a), cudaEventDestroy(t.b);
   if (ctx->graph_exec) cudaGraphExecDestroy(ctx->graph_exec);
   cudaEventDestroy(ctx->ev0), cudaEventDestroy(ctx->ev1);
@@ -399,12 +436,16 @@ void rayn_b200_destroy(RaynContext* ctx) {
 static int32_t validate_scene(RaynContext* ctx, const RaynSceneDesc* s) {
   if (!s) return fail(ctx, RAYN_ERR_INVALID_ARG, "scene is NULL");
   if (s->n_hitables < 1 || s->n_hitables > RAYN_MAX_HITABLES)
-    return fail(ctx, RAYN_ERR_INVALID_ARG, "n_hitables %d not in [1,%d]", s->n_hitables, RAYN_MAX_HITABLES);
+    return fail(ctx, RAYN_ERR_INVALID_ARG, "n_hitables %d not in [1,%d] (RAYN_MAX_HITABLES)", s->n_hitables, RAYN_MAX_HITABLES);
   if (s->n_materials < 1 || s->n_materials > RAYN_MAX_MATERIALS)
-    return fail(ctx, RAYN_ERR_INVALID_ARG, "n_materials %d not in [1,%d]", s->n_materials, RAYN_MAX_MATERIALS);
+    return fail(ctx, RAYN_ERR_INVALID_ARG, "n_materials %d not in [1,%d] (RAYN_MAX_MATERIALS)", s->n_materials, RAYN_MAX_MATERIALS);
   if (s->n_lights < 0 || s->n_lights > RAYN_MAX_LIGHTS)
-    return fail(ctx, RAYN_ERR_INVALID_ARG, "n_lights %d not in [0,%d]", s->n_lights, RAYN_MAX_LIGHTS);
+    return fail(ctx, RAYN_ERR_INVALID_ARG, "n_lights %d not in [0,%d] (RAYN_MAX_LIGHTS)", s->n_lights, RAYN_MAX_LIGHTS);
   if (!s->hitables || !s->materials || (s->n_lights && !s->lights)) return fail(ctx, RAYN_ERR_INVALID_ARG, "NULL scene array");
+  int n_sdf = 0;
+  for (int i = 0; i < s->n_hitables; ++i) n_sdf += s->hitables[i].kind != RAYN_HITABLE_SPHERE ? 1 : 0;
+  if (n_sdf > RAYN_MAX_SDF_HITABLES)
+    return fail(ctx, RAYN_ERR_INVALID_ARG, "%d SDF hitables, more than %d (RAYN_MAX_SDF_HITABLES)", n_sdf, RAYN_MAX_SDF_HITABLES);
   for (int i = 0; i < s->n_hitables; ++i) {
     const RaynHitable& h = s->hitables[i];
     if (h.kind < 0 || h.kind > RAYN_HITABLE_MANDELBULB) return fail(ctx, RAYN_ERR_INVALID_ARG, "hitable %d: bad kind %d", i, h.kind);
@@ -453,33 +494,78 @@ int32_t rayn_b200_upload_scene(RaynContext* ctx, const RaynSceneDesc* s) {
   if (!ctx) return fail(nullptr, RAYN_ERR_INVALID_ARG, "ctx is NULL");
   int32_t rc = validate_scene(ctx, s);
   if (rc) return rc;
+  ctx->has_scene = false;
+  const int nh = s->n_hitables, nm = s->n_materials, nl = s->n_lights;
+  ctx->h_hit.assign(s->hitables, s->hitables + nh);
+  ctx->h_mat.assign(s->materials, s->materials + nm);
+  // compact sphere / SDF lists in insertion order (DevScene)
+  std::vector<int32_t> sph_idx, sdf_idx, hit_ord(nh);
+  std::vector<float4> sph;
+  int sph_moving = 0;
+  for (int i = 0; i < nh; ++i) {
+    const RaynHitable& h = s->hitables[i];
+    if (h.kind == RAYN_HITABLE_SPHERE) {
+      hit_ord[i] = (int32_t)sph_idx.size();
+      sph_idx.push_back(i);
+      sph.push_back(make_float4(h.center[0], h.center[1], h.center[2], h.radius));
+      sph_moving |= (h.center_velocity[0] != 0.0f || h.center_velocity[1] != 0.0f || h.center_velocity[2] != 0.0f) ? 1 : 0;
+    } else {
+      hit_ord[i] = (int32_t)sdf_idx.size();
+      sdf_idx.push_back(i);
+    }
+  }
   DevScene& d = ctx->scene;
   memset(&d, 0, sizeof d);
-  d.n_hit = s->n_hitables;
-  d.n_mat = s->n_materials;
-  d.n_lights = s->n_lights;
+  d.n_hit = nh;
+  d.n_mat = nm;
+  d.n_lights = nl;
   d.one = 1.0f;
-  memcpy(d.hit, s->hitables, sizeof(RaynHitable) * s->n_hitables);
-  memcpy(d.mat, s->materials, sizeof(RaynMaterial) * s->n_materials);
-  if (s->n_lights) memcpy(d.light, s->lights, sizeof(RaynLight) * s->n_lights);
   d.cam = s->camera;
   d.vol = s->volume;
   d.rc = s->consts;
-  for (int i = 0; i < d.n_hit; ++i) {  // compact sphere / SDF lists in insertion order (DevScene)
-    const RaynHitable& h = d.hit[i];
-    if (h.kind == RAYN_HITABLE_SPHERE) {
-      d.sph_idx[d.n_sph] = i;
-      d.hit_ord[i] = d.n_sph;
-      d.sph[d.n_sph] = make_float4(h.center[0], h.center[1], h.center[2], h.radius);
-      d.sph_moving |= (h.center_velocity[0] != 0.0f || h.center_velocity[1] != 0.0f || h.center_velocity[2] != 0.0f) ? 1 : 0;
-      ++d.n_sph;
-    } else {
-      d.hit_ord[i] = d.n_sdf;
-      d.sdf_idx[d.n_sdf++] = i;
-    }
+  d.n_sph = (int32_t)sph_idx.size();
+  d.n_sdf = (int32_t)sdf_idx.size();
+  d.sph_moving = sph_moving;
+  ctx->tables = (ctx->flags & RAYN_FLAG_SCENE_TABLES) || nh > SCENE_INLINE_MAX || nm > SCENE_INLINE_MAX || nl > SCENE_INLINE_MAX;
+  if (!ctx->tables) {
+    memcpy(d.hit, s->hitables, sizeof(RaynHitable) * nh);
+    memcpy(d.mat, s->materials, sizeof(RaynMaterial) * nm);
+    if (nl) memcpy(d.light, s->lights, sizeof(RaynLight) * nl);
+    std::copy(sph_idx.begin(), sph_idx.end(), d.sph_idx);
+    std::copy(sdf_idx.begin(), sdf_idx.end(), d.sdf_idx);
+    std::copy(hit_ord.begin(), hit_ord.end(), d.hit_ord);
+    std::copy(sph.begin(), sph.end(), d.sph);
+  } else {
+    // one device block: the seven tables, each 256-byte aligned
+    size_t off[7], total = 0;
+    const size_t bytes[7] = {sizeof(RaynHitable) * nh, sizeof(RaynMaterial) * nm, sizeof(RaynLight) * nl, sizeof(int32_t) * sph_idx.size(),
+                             sizeof(int32_t) * sdf_idx.size(), sizeof(int32_t) * nh, sizeof(float4) * sph.size()};
+    const void* src[7] = {s->hitables, s->materials, s->lights, sph_idx.data(), sdf_idx.data(), hit_ord.data(), sph.data()};
+    for (int t = 0; t < 7; ++t) off[t] = total, total += (bytes[t] + 255) & ~(size_t)255;
+    std::vector<unsigned char> blob(total, 0);
+    for (int t = 0; t < 7; ++t)
+      if (bytes[t]) memcpy(blob.data() + off[t], src[t], bytes[t]);
+    CU(cudaSetDevice(ctx->device));
+    CU(cudaStreamSynchronize(ctx->stream));  // kernels still in flight may read the tables that are rewritten here
+    CU(regrow(&ctx->d_tables, &ctx->cap_tables, total));
+    CU(cudaMemcpyAsync(ctx->d_tables, blob.data(), total, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    TableScene& t = ctx->tscene;
+    memset(&t, 0, sizeof t);
+    t.n_hit = d.n_hit, t.n_mat = d.n_mat, t.n_lights = d.n_lights, t.one = d.one;
+    t.hit.p = (const RaynHitable*)(ctx->d_tables + off[0]);
+    t.mat.p = (const RaynMaterial*)(ctx->d_tables + off[1]);
+    t.light.p = (const RaynLight*)(ctx->d_tables + off[2]);
+    t.cam = d.cam, t.vol = d.vol, t.rc = d.rc;
+    t.n_sph = d.n_sph, t.n_sdf = d.n_sdf, t.sph_moving = d.sph_moving;
+    t.sph_idx.p = (const int32_t*)(ctx->d_tables + off[3]);
+    t.sdf_idx.p = (const int32_t*)(ctx->d_tables + off[4]);
+    t.hit_ord.p = (const int32_t*)(ctx->d_tables + off[5]);
+    t.sph.p = (const float4*)(ctx->d_tables + off[6]);
   }
-  for (int i = 0; i < d.n_hit; ++i)
-    ctx->sdf_var[i] = d.hit[i].kind == RAYN_HITABLE_SPHERE ? -1 : sdf_variant(d.hit[i], !(ctx->flags & RAYN_FLAG_NO_DIV3) && div3_verified(ctx, d.hit[i]));
+  ++ctx->scene_gen;
+  for (int i = 0; i < nh; ++i)
+    ctx->sdf_var[i] = s->hitables[i].kind == RAYN_HITABLE_SPHERE ? -1 : sdf_variant(s->hitables[i], !(ctx->flags & RAYN_FLAG_NO_DIV3) && div3_verified(ctx, s->hitables[i]));
   ctx->has_scene = true;
   return RAYN_OK;
 }
@@ -613,37 +699,41 @@ static int32_t render_enqueue(RaynContext* ctx, const RaynFrameDesc* f, const Ra
     dev_planes_out->space = RAYN_MEM_DEVICE;
   }
 
-  int n_sdf = 0;
-  int sdf_idx[RAYN_MAX_HITABLES];
+  const std::vector<RaynHitable>& hit = ctx->h_hit;
+  std::vector<int> sdf_idx;
   for (int i = 0; i < n_hit; ++i)
-    if (ctx->scene.hit[i].kind != RAYN_HITABLE_SPHERE) sdf_idx[n_sdf++] = i;
+    if (hit[i].kind != RAYN_HITABLE_SPHERE) sdf_idx.push_back(i);
+  const int n_sdf = (int)sdf_idx.size();
   const bool simple = (ctx->flags & RAYN_FLAG_SIMPLE_MARCH) != 0;
+  if (simple && ctx->tables)
+    return fail(ctx, RAYN_ERR_UNSUPPORTED, "scenes beyond %d hitables, materials or lights are not supported by the legacy test kernels", SCENE_INLINE_MAX);
   bool motion = false;  // time-varying sphere centres need the packet's lane-0 time: only the product kernels plumb it
   for (int i = 0; i < n_hit; ++i)
-    motion |= ctx->scene.hit[i].kind == RAYN_HITABLE_SPHERE && (ctx->scene.hit[i].center_velocity[0] != 0.0f || ctx->scene.hit[i].center_velocity[1] != 0.0f ||
-                                                                 ctx->scene.hit[i].center_velocity[2] != 0.0f);
+    motion |= hit[i].kind == RAYN_HITABLE_SPHERE && (hit[i].center_velocity[0] != 0.0f || hit[i].center_velocity[1] != 0.0f || hit[i].center_velocity[2] != 0.0f);
   if (motion && simple) return fail(ctx, RAYN_ERR_UNSUPPORTED, "time-varying sphere centres are not supported by the legacy test kernels");
   // leading analytic spheres run inside raygen / shade_post (rt_kernels.cuh::fold_head); -1 = not folded (moving spheres need
   // the extend packet's lane-0 time; the legacy test kernels do the whole fold themselves)
   int fold_pre = -1;
   if (!motion && !simple) {
     fold_pre = 0;
-    while (fold_pre < n_hit && ctx->scene.hit[fold_pre].kind == RAYN_HITABLE_SPHERE) ++fold_pre;
+    while (fold_pre < n_hit && hit[fold_pre].kind == RAYN_HITABLE_SPHERE) ++fold_pre;
   }
   // Scenes of the shape [spheres] Mandelbox [spheres] (setup.rs) fold ALL analytic spheres into the producing kernel and march
   // the SDF last, against the nearest sphere: one gather of every live ray per depth less (k_extend_spheres was 2 % of a
   // config-3 frame) and shorter marches for rays that end on an emitter.  The result is the reference's fold bit for bit
   // (proof in rt_kernels.cuh at k_extend_march: it needs a distance estimator that is never negative, i.e. the Mandelbox -
   // sqrt(m) / |dr| - so that a march's t never decreases, and the first-index-wins tie rule, which the kernel applies).
-  const bool fold_all = fold_pre >= 0 && n_sdf == 1 && ctx->scene.hit[sdf_idx[0]].kind == RAYN_HITABLE_MANDELBOX && !(ctx->flags & RAYN_FLAG_NO_FOLD_ALL);
+  const bool fold_all = fold_pre >= 0 && n_sdf == 1 && hit[sdf_idx[0]].kind == RAYN_HITABLE_MANDELBOX && !(ctx->flags & RAYN_FLAG_NO_FOLD_ALL);
   const int n_fold = fold_all ? ctx->scene.n_sph : fold_pre;  // leading spheres are the first fold_pre entries of the compact sphere list
   const bool volume_on = ctx->scene.vol.has_scattering != 0 && ctx->scene.n_lights > 0;
   const int ns = volume_on ? 4 * (1 + vm) : 4;               // light samples per path per depth
   const int seg_per_path = simple ? 0 : ns * n_sdf;          // worst case shadow segments per path per depth, all SDF queues
   const int lc_ns = simple ? 0 : ns;                         // stored light contributions per path per depth
+  const int maxk = ctx->tables ? TableScene::kMaxHit : DevScene::kMaxHit;  // keys of the bin kernels, row stride of the bin tables
+  const RaynContext::Occ& occ = ctx->occ[ctx->tables ? 1 : 0];
 
   // pass size: as many tiles as the requested path budget AND free device memory allow
-  const size_t bpp = pass_bytes_per_path(R, QS, seg_per_path, lc_ns);
+  const size_t bpp = pass_bytes_per_path(R, QS, seg_per_path, lc_ns, maxk);
   size_t free_b = 0, total_b = 0;
   CU(cudaMemGetInfo(&free_b, &total_b));
   const size_t budget = (size_t)((double)(free_b + ctx->pass_bytes) * 0.90);
@@ -654,7 +744,7 @@ static int32_t render_enqueue(RaynContext* ctx, const RaynFrameDesc* f, const Ra
   tiles_per_pass = std::min(tiles_per_pass, 65535);
   tiles_per_pass = std::min<int>(tiles_per_pass, (int)std::max<size_t>(my_tiles.size(), 1));
   int32_t rc;
-  while ((rc = ensure_pass(ctx, tiles_per_pass, R, QS, seg_per_path, n_sdf, lc_ns)) == RAYN_ERR_OOM && tiles_per_pass > 1)
+  while ((rc = ensure_pass(ctx, tiles_per_pass, R, QS, seg_per_path, n_sdf, lc_ns, maxk)) == RAYN_ERR_OOM && tiles_per_pass > 1)
     tiles_per_pass = (tiles_per_pass + 1) / 2;  // fragmentation / another tenant: retry with half the pass
   if (rc) return rc;
   PassBufs pb = ctx->pb;
@@ -680,6 +770,10 @@ static int32_t render_enqueue(RaynContext* ctx, const RaynFrameDesc* f, const Ra
     PassBufs kpb = pb;
     kpb.n_tiles = (int)my_tiles.size();
     key = fnv1a(1469598103934665603ull, &ctx->scene, sizeof ctx->scene);
+    if (ctx->tables) {  // the launches carry only the tables' pointers: the upload count stands for their contents
+      key = fnv1a(key, &ctx->tscene, sizeof ctx->tscene);
+      key = fnv1a(key, &ctx->scene_gen, sizeof ctx->scene_gen);
+    }
     key = fnv1a(key, &fr, sizeof fr);
     key = fnv1a(key, &kpb, sizeof kpb);
     float* planes4[4] = {p_color, p_alpha, p_bg, p_normal};
@@ -695,22 +789,17 @@ static int32_t render_enqueue(RaynContext* ctx, const RaynFrameDesc* f, const Ra
     }
   }
   std::vector<int> h_nslots, h_slots;
-  for (size_t first = 0; first < my_tiles.size() && !replayed; first += tiles_per_pass) {
-    const int nt = (int)std::min<size_t>(tiles_per_pass, my_tiles.size() - first);
-    pb.n_tiles = nt;
-    CU(cudaMemcpyAsync(ctx->d_tile_ids, my_tiles.data() + first, nt * sizeof(int), cudaMemcpyHostToDevice, st));
-    if (use_graph) {
-      CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-      capturing = true;
-    }
-    ctx->stats.passes++;
+  // the kernel sequence of one pass of nt tiles starting at my_tiles[first], for either scene type
+  auto run_pass = [&](const auto& sc, const int nt, const size_t first) -> int32_t {
+    using S = std::decay_t<decltype(sc)>;
     const dim3 g_paths((R + 255) / 256, nt), g_shade((QS + 127) / 128, nt);
+    (void)g_shade;
     // resident grids (one wave) of the kernels that stride over a work list (k_scan_slots / k_scan_live), capped by the list's upper bound
     const int64_t max_blocks = (int64_t)nt * ((QS + SLOT_BLOCK - 1) / SLOT_BLOCK);
-    auto resident = [&](int occ) { return (unsigned)std::max<int64_t>(1, std::min<int64_t>((int64_t)ctx->n_sm * occ, max_blocks)); };
+    auto resident = [&](int o) { return (unsigned)std::max<int64_t>(1, std::min<int64_t>((int64_t)ctx->n_sm * o, max_blocks)); };
     const int nseg = (QS + SEG_SLOTS - 1) / SEG_SLOTS;  // segments per tile of the queue kernels
     timed_begin(ctx, RAYN_K_RAYGEN);
-    k_raygen<<<g_paths, 256, 0, st>>>(ctx->scene, fr, pb, n_fold);
+    k_raygen<S><<<g_paths, 256, 0, st>>>(sc, fr, pb, n_fold);
     timed_end(ctx, RAYN_K_RAYGEN);
     for (int depth = 0; depth <= mb; ++depth) {
       const Thr thr = make_thr(ctx->scene.cam, depth);
@@ -729,10 +818,11 @@ static int32_t render_enqueue(RaynContext* ctx, const RaynFrameDesc* f, const Ra
         int k = fold_pre >= 0 ? fold_pre : 0, first_kernel = fold_pre >= 0 ? 0 : 1, n_march = 0;
         while (k < n_hit || first_kernel) {
           int e = k;
-          while (e < n_hit && ctx->scene.hit[e].kind == RAYN_HITABLE_SPHERE) ++e;
+          while (e < n_hit && hit[e].kind == RAYN_HITABLE_SPHERE) ++e;
           if ((e > k || first_kernel) && !fold_all) {
+            const int run = (int)(std::lower_bound(sdf_idx.begin(), sdf_idx.end(), k) - sdf_idx.begin());  // SDFs before the run
             timed_begin(ctx, RAYN_K_EXTEND_SPHERES);
-            k_extend_spheres<<<resident(ctx->occ_sph), EXT_BATCH, 0, st>>>(ctx->scene, pb, k, e, first_kernel, motion ? 1 : 0, ctx->d_batch_prefix, ctx->d_work_ctr + WC_SPHERES + k);
+            k_extend_spheres<S><<<resident(occ.sph), EXT_BATCH, 0, st>>>(sc, pb, k, e, first_kernel, motion ? 1 : 0, ctx->d_batch_prefix, ctx->d_work_ctr + WC_SPHERES + run);
             timed_end(ctx, RAYN_K_EXTEND_SPHERES);
             first_kernel = 0;
           }
@@ -740,7 +830,7 @@ static int32_t render_enqueue(RaynContext* ctx, const RaynFrameDesc* f, const Ra
             if (n_march++ > 0) CU(cudaMemsetAsync(ctx->d_work_ctr + WC_EXTEND, 0, sizeof(int), st));
             const int v = ctx->sdf_var[e];
             timed_begin(ctx, RAYN_K_EXTEND);
-            DISPATCH_SDFV(v, (k_extend_march<V><<<ctx->n_sm * ctx->occ_ext[v], EXT_T, 0, st>>>(ctx->scene, pb, thr, e, fold_all ? 1 : 0, ctx->d_batch_prefix, ctx->d_work_ctr + WC_EXTEND)));
+            DISPATCH_SDFV(v, (k_extend_march<V, S><<<ctx->n_sm * occ.ext[v], EXT_T, 0, st>>>(sc, pb, thr, e, fold_all ? 1 : 0, ctx->d_batch_prefix, ctx->d_work_ctr + WC_EXTEND)));
             timed_end(ctx, RAYN_K_EXTEND);
             ++e;
           }
@@ -748,9 +838,12 @@ static int32_t render_enqueue(RaynContext* ctx, const RaynFrameDesc* f, const Ra
         }
       }
       timed_begin(ctx, RAYN_K_BIN);
-      k_bin_count<<<dim3(nseg, nt), BIN_T, 0, st>>>(pb, n_hit, nseg);
-      k_bin_scatter<<<dim3(nseg, nt), BIN_T, 0, st>>>(pb, n_hit, nseg);
-      if (!simple) k_scan_slots<<<1, SCAN_T, 0, st>>>(ctx->scene, pb);  // work lists of k_normals / k_shade_pre / k_shade_post
+      k_bin_count<S::kMaxHit><<<dim3(nseg, nt), BIN_T, 0, st>>>(pb, n_hit, nseg);
+      if (ctx->tables)
+        k_bin_scatter_tables<<<dim3(nseg, nt), BINB_T, 0, st>>>(pb, n_hit, nseg);
+      else
+        k_bin_scatter<<<dim3(nseg, nt), BIN_T, 0, st>>>(pb, n_hit, nseg);
+      if (!simple) k_scan_slots<S><<<1, SCAN_T, 0, st>>>(sc, pb);  // work lists of k_normals / k_shade_pre / k_shade_post
       timed_end(ctx, RAYN_K_BIN, simple ? 2 : 3);
       if (ctx->qlog_enabled) {
         h_nslots.resize(nt);
@@ -768,27 +861,27 @@ static int32_t render_enqueue(RaynContext* ctx, const RaynFrameDesc* f, const Ra
       if (!simple) {
         // get_shading_info of the SDF hitables whose material is shaded (receives light, or volumetrics sample along the ray)
         for (int j = 0; j < n_sdf; ++j) {
-          const RaynHitable& h = ctx->scene.hit[sdf_idx[j]];
-          const int mk = ctx->scene.mat[h.material].kind;
+          const RaynHitable& h = hit[sdf_idx[j]];
+          const int mk = ctx->h_mat[h.material].kind;
           if (!(mk == RAYN_MATERIAL_LAMBERTIAN || mk == RAYN_MATERIAL_DIELECTRIC || volume_on)) continue;
           const int v = ctx->sdf_var[sdf_idx[j]];
           timed_begin(ctx, RAYN_K_NORMALS);
-          DISPATCH_SDFV(v, (k_normals<V><<<resident(ctx->occ_nrm[v]), SLOT_BLOCK, 0, st>>>(ctx->scene, pb, thr, sdf_idx[j], j, ctx->d_work_ctr + WC_NORMALS + j)));
+          DISPATCH_SDFV(v, (k_normals<V, S><<<resident(occ.nrm[v]), SLOT_BLOCK, 0, st>>>(sc, pb, thr, sdf_idx[j], j, ctx->d_work_ctr + WC_NORMALS + j)));
           timed_end(ctx, RAYN_K_NORMALS);
         }
         timed_begin(ctx, RAYN_K_SHADE_PRE);
-        k_shade_pre<<<resident(ctx->occ_pre), SLOT_BLOCK, 0, st>>>(ctx->scene, fr, pb, depth, thr, ctx->d_work_ctr + WC_PRE);
+        k_shade_pre<S><<<resident(occ.pre), SLOT_BLOCK, 0, st>>>(sc, fr, pb, depth, thr, ctx->d_work_ctr + WC_PRE);
         timed_end(ctx, RAYN_K_SHADE_PRE);
         if (ctx->scene.n_lights > 0) {
           for (int j = 0; j < n_sdf; ++j) {
             const int v = ctx->sdf_var[sdf_idx[j]];
             timed_begin(ctx, RAYN_K_SHADOW);
-            DISPATCH_SDFV(v, (k_shadow<V><<<ctx->n_sm * ctx->occ_shd[v], SHD_T, 0, st>>>(ctx->scene, pb, sdf_idx[j], j, ctx->d_work_ctr + WC_SHADOW + j)));
+            DISPATCH_SDFV(v, (k_shadow<V, S><<<ctx->n_sm * occ.shd[v], SHD_T, 0, st>>>(sc, pb, sdf_idx[j], j, ctx->d_work_ctr + WC_SHADOW + j)));
             timed_end(ctx, RAYN_K_SHADOW);
           }
         }
         timed_begin(ctx, RAYN_K_SHADE_POST);
-        k_shade_post<<<resident(ctx->occ_post), SLOT_BLOCK, 0, st>>>(ctx->scene, fr, pb, depth, n_fold, ctx->d_work_ctr + WC_POST);
+        k_shade_post<S><<<resident(occ.post), SLOT_BLOCK, 0, st>>>(sc, fr, pb, depth, n_fold, ctx->d_work_ctr + WC_POST);
         timed_end(ctx, RAYN_K_SHADE_POST);
       } else {
 #ifdef RAYN_LEGACY_KERNELS
@@ -807,6 +900,18 @@ static int32_t render_enqueue(RaynContext* ctx, const RaynFrameDesc* f, const Ra
     timed_begin(ctx, RAYN_K_RESOLVE);
     k_resolve<<<dim3((f->tile_w * f->tile_h + wpc - 1) / wpc, nt), wpc * 32, res_smem, st>>>(fr, pb, p_color, p_alpha, p_bg, p_normal, np, wpc, slot_bits, depth_bits);
     timed_end(ctx, RAYN_K_RESOLVE);
+    return RAYN_OK;
+  };
+  for (size_t first = 0; first < my_tiles.size() && !replayed; first += tiles_per_pass) {
+    const int nt = (int)std::min<size_t>(tiles_per_pass, my_tiles.size() - first);
+    pb.n_tiles = nt;
+    CU(cudaMemcpyAsync(ctx->d_tile_ids, my_tiles.data() + first, nt * sizeof(int), cudaMemcpyHostToDevice, st));
+    if (use_graph) {
+      CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+      capturing = true;
+    }
+    ctx->stats.passes++;
+    if ((rc = ctx->tables ? run_pass(ctx->tscene, nt, first) : run_pass(ctx->scene, nt, first))) return rc;
     if (capturing) {
       cudaGraph_t graph = nullptr;
       CU(cudaStreamEndCapture(st, &graph));
@@ -1297,7 +1402,10 @@ int32_t rayn_b200_kat_occluded(RaynContext* ctx, int64_t n, const float* start3,
   float* de = tmp.up(end3, 3 * n, &e);
   float* dout = tmp.up<float>(nullptr, n, &e);
   CU(e);
-  k_kat_occluded<<<blocks, 128, 0, ctx->stream>>>(ctx->scene, n, ds, de, dout);
+  if (ctx->tables)
+    k_kat_occluded<<<blocks, 128, 0, ctx->stream>>>(ctx->tscene, n, ds, de, dout);
+  else
+    k_kat_occluded<<<blocks, 128, 0, ctx->stream>>>(ctx->scene, n, ds, de, dout);
   KAT_EPILOGUE(out, dout, n, float)
   return RAYN_OK;
 }
@@ -1311,7 +1419,10 @@ int32_t rayn_b200_kat_closest_hit(RaynContext* ctx, int32_t depth, int64_t n, co
   float* dt = tmp.up<float>(nullptr, n, &e);
   int* dobj = tmp.up<int>(nullptr, n, &e);
   CU(e);
-  k_kat_closest_hit<<<blocks, 128, 0, ctx->stream>>>(ctx->scene, make_thr(ctx->scene.cam, depth), n, dor, ddi, dt, dobj);
+  if (ctx->tables)
+    k_kat_closest_hit<<<blocks, 128, 0, ctx->stream>>>(ctx->tscene, make_thr(ctx->scene.cam, depth), n, dor, ddi, dt, dobj);
+  else
+    k_kat_closest_hit<<<blocks, 128, 0, ctx->stream>>>(ctx->scene, make_thr(ctx->scene.cam, depth), n, dor, ddi, dt, dobj);
   KAT_EPILOGUE(out_t, dt, n, float)
   CU(cudaMemcpy(out_obj, dobj, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost));
   return RAYN_OK;

@@ -105,22 +105,72 @@ RT_D float f_schlick(float cosv, float f0) { return f0 + (1.0f - f0) * dm::powi5
 // ------------------------------------------------------------------------------------------
 // Scene as a kernel-parameter block (constant bank: warp-uniform operands cost no load)
 // ------------------------------------------------------------------------------------------
+// Scenes with at most SCENE_INLINE_MAX hitables, materials and lights ride in the parameter block itself (DevScene); larger
+// ones keep the same tables in device memory (TableScene).  The kernels are templates on the scene type and read both
+// through the same expressions (sc.hit[i], sc.sph[k], ...).
+#define SCENE_INLINE_MAX 16
 struct DevScene {
+  static constexpr int kMaxHit = SCENE_INLINE_MAX;  // row stride - 1 of the per-tile bin tables (PassBufs::bin_start)
   int32_t n_hit, n_mat, n_lights;
   float one;  // 1.0f, set at upload: a multiplier the compiler cannot constant-fold (rt_sdf2.cuh::muladd2)
-  RaynHitable hit[RAYN_MAX_HITABLES];
-  RaynMaterial mat[RAYN_MAX_MATERIALS];
-  RaynLight light[RAYN_MAX_LIGHTS];
+  RaynHitable hit[SCENE_INLINE_MAX];
+  RaynMaterial mat[SCENE_INLINE_MAX];
+  RaynLight light[SCENE_INLINE_MAX];
   RaynCamera cam;
   RaynVolume vol;
   RaynRenderConsts rc;
-  // derived at upload (api.cu::derive_scene_tables): the analytic spheres and the SDF hitables as compact lists in insertion
-  // order, so that the shading kernels neither walk all hitables testing `kind` nor index 40-byte descriptors per lane
+  // derived at upload (api.cu::rayn_b200_upload_scene): the analytic spheres and the SDF hitables as compact lists in
+  // insertion order, so that the shading kernels neither walk all hitables testing `kind` nor index 40-byte descriptors per lane
   int32_t n_sph, n_sdf, sph_moving, pad_;
-  int32_t sph_idx[RAYN_MAX_HITABLES];  // hitable index of sphere k
-  int32_t sdf_idx[RAYN_MAX_HITABLES];  // hitable index of SDF ordinal j
-  int32_t hit_ord[RAYN_MAX_HITABLES];  // hitable i is the hit_ord[i]-th sphere / SDF
-  float4 sph[RAYN_MAX_HITABLES];       // centre.xyz, radius of sphere k (a moving sphere keeps its t = 0 centre here)
+  int32_t sph_idx[SCENE_INLINE_MAX];  // hitable index of sphere k
+  int32_t sdf_idx[SCENE_INLINE_MAX];  // hitable index of SDF ordinal j
+  int32_t hit_ord[SCENE_INLINE_MAX];  // hitable i is the hit_ord[i]-th sphere / SDF
+  float4 sph[SCENE_INLINE_MAX];       // centre.xyz, radius of sphere k (a moving sphere keeps its t = 0 centre here)
+};
+
+// One element of a read-only device table through the non-coherent path (LDG.CONSTANT), in the widest loads its size allows.
+template <class T>
+RT_D T ldg_elem(const T* p) {
+  static_assert(sizeof(T) % 4 == 0, "table elements are made of 32-bit words");
+  if constexpr (sizeof(T) % 16 == 0) {
+    union { T t; float4 w[sizeof(T) / 16]; } u;
+#pragma unroll
+    for (int i = 0; i < (int)(sizeof(T) / 16); ++i) u.w[i] = __ldg(reinterpret_cast<const float4*>(p) + i);
+    return u.t;
+  } else if constexpr (sizeof(T) % 8 == 0) {
+    union { T t; float2 w[sizeof(T) / 8]; } u;
+#pragma unroll
+    for (int i = 0; i < (int)(sizeof(T) / 8); ++i) u.w[i] = __ldg(reinterpret_cast<const float2*>(p) + i);
+    return u.t;
+  } else {
+    union { T t; float w[sizeof(T) / 4]; } u;
+#pragma unroll
+    for (int i = 0; i < (int)(sizeof(T) / 4); ++i) u.w[i] = __ldg(reinterpret_cast<const float*>(p) + i);
+    return u.t;
+  }
+}
+template <class T>
+struct LdgTable {
+  const T* p;
+  RT_D T operator[](int i) const { return ldg_elem(p + i); }
+};
+// The scene of the large-scene path: DevScene's fields, its arrays as tables in device memory that the context owns
+// (written once per upload, api.cu).  Loads that differ per lane (the hit object's descriptor, its material, a light) and
+// the loops every lane of a warp walks in the same order (sphere lists) both go through LDG: the uniform ones are one
+// broadcast transaction per warp, served from L1 after the first warp of the SM.
+struct TableScene {
+  static constexpr int kMaxHit = RAYN_MAX_HITABLES;
+  int32_t n_hit, n_mat, n_lights;
+  float one;
+  LdgTable<RaynHitable> hit;
+  LdgTable<RaynMaterial> mat;
+  LdgTable<RaynLight> light;
+  RaynCamera cam;
+  RaynVolume vol;
+  RaynRenderConsts rc;
+  int32_t n_sph, n_sdf, sph_moving, pad_;
+  LdgTable<int32_t> sph_idx, sdf_idx, hit_ord;
+  LdgTable<float4> sph;
 };
 
 // the `hit_threshold_at` closure of film.rs:540-551
@@ -367,7 +417,8 @@ RT_D float sphere_hit_static(const float4 cr, f3 ro, f3 rd, float t_max) {
 }
 
 // HitableStore::add_hits fold, hitable.rs:177-198
-RT_D void closest_hit(const DevScene& sc, f3 o, f3 d, Thr thr, float* out_t, int* out_obj, int* evals, float time0 = 0.0f) {
+template <class Scn>
+RT_D void closest_hit(const Scn& sc, f3 o, f3 d, Thr thr, float* out_t, int* out_obj, int* evals, float time0 = 0.0f) {
   float closest = sc.rc.world_radius * 2.0f;  // film.rs:556
   int id = -1;
   for (int i = 0; i < sc.n_hit; ++i) {
@@ -385,7 +436,8 @@ RT_D void closest_hit(const DevScene& sc, f3 o, f3 d, Thr thr, float* out_t, int
 // HitableStore::test_occluded, hitable.rs:164-168.  The reference multiplies occluded() in
 // {0,1} over ALL hitables; a product of exact 0/1 floats is 0 iff any factor is 0, so the
 // cheap analytic spheres are tested first and the march is skipped once occlusion is known.
-RT_D float test_occluded(const DevScene& sc, f3 start, f3 end, int* evals, float time0 = 0.0f) {
+template <class Scn>
+RT_D float test_occluded(const Scn& sc, f3 start, f3 end, int* evals, float time0 = 0.0f) {
   for (int i = 0; i < sc.n_hit; ++i)
     if (sc.hit[i].kind == RAYN_HITABLE_SPHERE && sphere_occluded(sc.hit[i], start, end, time0) == 0.0f) return 0.0f;
   for (int i = 0; i < sc.n_hit; ++i)

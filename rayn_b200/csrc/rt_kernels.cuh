@@ -56,7 +56,7 @@ struct PassBufs {
   int* q_shade;
   int* n_live;     // [n_tiles]
   int* n_slots;    // [n_tiles]
-  int* bin_start;  // [n_tiles*(RAYN_MAX_HITABLES+1)]
+  int* bin_start;  // [n_tiles*(Scn::kMaxHit+1)]: bin starts of every hitable, row stride by scene type (rt_device.cuh)
   unsigned long long* counters;  // [8] stats
   // shading split (normals -> pre -> persistent shadow march -> post)
   float4* nrm;        // [paths] shading normal.xyz, offset_by of the current depth (hitable.rs:21-28)
@@ -64,15 +64,15 @@ struct PassBufs {
   // shadow segments of the current depth, one queue per SDF hitable (ordinal j): entries [j*seg_cap, j*seg_cap + seg_count[j])
   float4* seg_a;      // start.xyz, max_dist
   float4* seg_b;      // dir.xyz, bits(path index g << 4 | light-sample bit)
-  int* seg_count;     // [RAYN_MAX_HITABLES] segments pushed this depth, per SDF ordinal
+  int* seg_count;     // [RAYN_MAX_SDF_HITABLES] segments pushed this depth, per SDF ordinal
   long long seg_cap;  // capacity of ONE queue
   float4* lc_c;       // [paths * lc_ns] unoccluded light contribution c.xyz and its denominator (pdf), per light sample of this depth
   float* lc_t;        // [paths * 8] volume rounds only: transmission to the scatter point (integrator.rs:122-126)
   int lc_ns;          // light samples per path per depth: 4, or 4 * (1 + vm) with volumetrics
-  int* seg_cnt;       // [n_tiles * nseg * RAYN_MAX_HITABLES] scratch of the segmented queue kernels (k_bin_*, k_compact_*)
+  int* seg_cnt;       // [n_tiles * nseg * Scn::kMaxHit] scratch of the segmented queue kernels (k_bin_*, k_compact_*)
   // work lists of the slot-parallel kernels (k_scan_slots): row 0 = 128-slot blocks of every tile's shading queue, row 1 + j =
   // 128-slot blocks of the bin of SDF ordinal j; each row is an exclusive prefix over the tiles with the total at [n_tiles]
-  int* slot_prefix;   // [(1 + RAYN_MAX_HITABLES) * prefix_stride]
+  int* slot_prefix;   // [(1 + RAYN_MAX_SDF_HITABLES) * prefix_stride]
   int prefix_stride;  // >= n_tiles + 1
 };
 
@@ -80,9 +80,10 @@ enum { CNT_EXTEND_RAYS = 0, CNT_SHADE_LANES = 1, CNT_SHADOW_RAYS = 2, CNT_EVALS_
        CNT_BULB_ITERS_EXTEND = 5, CNT_BULB_ITERS_SHADOW = 6, CNT_EVALS_NORMALS = 7, CNT_TRIPS_EXTEND = 8, CNT_TRIPS_SHADOW = 9, CNT_TOTAL = 10 };  // Mandelbulb iterations actually run (the count is data dependent)
 
 // global work counters of the persistent kernels (RaynContext::d_work_ctr), zeroed by k_scan_live every depth
-enum { WC_EXTEND = 0, WC_SHADOW = 1 /* + SDF ordinal */, WC_SEG_COUNT = 1 + RAYN_MAX_HITABLES /* + SDF ordinal */,
-       WC_PRE = 1 + 2 * RAYN_MAX_HITABLES, WC_POST = WC_PRE + 1, WC_NORMALS = WC_POST + 1 /* + SDF ordinal */,
-       WC_SPHERES = WC_NORMALS + RAYN_MAX_HITABLES /* + first hitable of the run */, WC_TOTAL = WC_SPHERES + RAYN_MAX_HITABLES };
+// (a run of spheres is numbered by the SDF hitables before it: runs are separated by SDFs, so there are at most 1 + n_sdf)
+enum { WC_EXTEND = 0, WC_SHADOW = 1 /* + SDF ordinal */, WC_SEG_COUNT = 1 + RAYN_MAX_SDF_HITABLES /* + SDF ordinal */,
+       WC_PRE = 1 + 2 * RAYN_MAX_SDF_HITABLES, WC_POST = WC_PRE + 1, WC_NORMALS = WC_POST + 1 /* + SDF ordinal */,
+       WC_SPHERES = WC_NORMALS + RAYN_MAX_SDF_HITABLES /* + SDFs before the run */, WC_TOTAL = WC_SPHERES + RAYN_MAX_SDF_HITABLES + 1 };
 
 #define TERM_NONE 0u
 #define TERM_COLOR 1u
@@ -132,7 +133,8 @@ RT_D void warp_add(unsigned long long* ctr, int v) {  // full warp; one REDUX in
 // the kernel that PRODUCES the ray (origin and direction are in registers there), which removes one gather of every live
 // ray per depth.  Static spheres only: a moving sphere is evaluated at the time of lane 0 of the extend packet, which is
 // not known before compaction (k_extend_spheres handles that case).
-RT_D void fold_head(const DevScene& sc, int n_fold, f3 o, f3 d, float* closest, int* id) {
+template <class Scn>
+RT_D void fold_head(const Scn& sc, int n_fold, f3 o, f3 d, float* closest, int* id) {
   float c = sc.rc.world_radius * 2.0f;
   int best = -1;
   for (int k = 0; k < n_fold; ++k) {
@@ -149,7 +151,8 @@ RT_D void fold_head(const DevScene& sc, int n_fold, f3 o, f3 d, float* closest, 
 // ------------------------------------------------------------------------------------------
 // K1 raygen: film.rs:456-529 + sample_uv :695-709 + camera.rs get_rays
 // ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) k_raygen(const __grid_constant__ DevScene sc, const DevFrame fr, const PassBufs pb, const int pre_n) {
+template <class Scn>
+__global__ void __launch_bounds__(256) k_raygen(const __grid_constant__ Scn sc, const DevFrame fr, const PassBufs pb, const int pre_n) {
   const int ts = blockIdx.y;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   const TileGeom tg = tile_geom(fr, pb.tile_ids[ts]);
@@ -183,6 +186,7 @@ __global__ void __launch_bounds__(256) k_raygen(const __grid_constant__ DevScene
   pb.term[g] = 0u;
   pb.q_live[g] = i;
 }
+template __global__ void k_raygen<DevScene>(const __grid_constant__ DevScene, const DevFrame, const PassBufs, const int);
 
 // ------------------------------------------------------------------------------------------
 // K3 bin+pad: HitStore::add_hit / process_hits (hitable.rs:90-133).  Stable partition of a
@@ -196,13 +200,15 @@ __global__ void __launch_bounds__(256) k_raygen(const __grid_constant__ DevScene
 // of its frame here.  A tile's live list is cut into SEG_SLOTS-ray segments; k_bin_count leaves per-segment per-object counts in
 // HBM, k_bin_scatter turns them into the segment's write cursors and scatters.  The partition stays stable (segments are in
 // order, a segment is scattered in order), so the queue is the same as the single-CTA one, bit for bit.
+// MAXK = the scene type's kMaxHit: the number of keys, and the row stride of seg_cnt
+template <int MAXK>
 __global__ void __launch_bounds__(BIN_T) k_bin_count(const PassBufs pb, const int n_hit, const int nseg) {
   const int seg = blockIdx.x, ts = blockIdx.y, tid = threadIdx.x, lane = tid & 31;
   const int n = pb.n_live[ts];
-  __shared__ int cnt[RAYN_MAX_HITABLES];
+  __shared__ int cnt[MAXK];
   const int* __restrict__ qk = pb.q_key + (size_t)ts * pb.R;  // per path
   const int* __restrict__ ql = pb.q_live + (size_t)ts * pb.R;
-  if (tid < RAYN_MAX_HITABLES) cnt[tid] = 0;
+  if (tid < MAXK) cnt[tid] = 0;
   if (tid == 0 && seg == 0 && n) atomicAdd(pb.counters + CNT_EXTEND_RAYS, (unsigned long long)n);  // rays through the closest-hit stage
   __syncthreads();
   const int lo = seg * SEG_SLOTS, hi = min(n, lo + SEG_SLOTS);
@@ -213,19 +219,20 @@ __global__ void __launch_bounds__(BIN_T) k_bin_count(const PassBufs pb, const in
     if (key >= 0 && (m & ((1u << lane) - 1)) == 0) atomicAdd(&cnt[key], __popc(m));
   }
   __syncthreads();
-  if (tid < n_hit) pb.seg_cnt[((size_t)ts * nseg + seg) * RAYN_MAX_HITABLES + tid] = cnt[tid];
+  if (tid < n_hit) pb.seg_cnt[((size_t)ts * nseg + seg) * MAXK + tid] = cnt[tid];
 }
+template __global__ void k_bin_count<SCENE_INLINE_MAX>(const PassBufs, const int, const int);
 __global__ void __launch_bounds__(BIN_T) k_bin_scatter(const PassBufs pb, const int n_hit, const int nseg) {
   const int seg = blockIdx.x, ts = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   constexpr int NW = BIN_T / 32;
   const int n = pb.n_live[ts];
   const int lo = seg * SEG_SLOTS, hi = min(n, lo + SEG_SLOTS);
   if (lo >= n && seg > 0) return;  // nothing to scatter; segment 0 still publishes the (possibly empty) bin table
-  __shared__ int cnt[RAYN_MAX_HITABLES];        // whole-tile counts
-  __shared__ int before[RAYN_MAX_HITABLES];     // counts of the segments before this one
-  __shared__ int start[RAYN_MAX_HITABLES + 1];
-  __shared__ int running[2][RAYN_MAX_HITABLES];
-  __shared__ int wcnt[2][NW][RAYN_MAX_HITABLES];
+  __shared__ int cnt[SCENE_INLINE_MAX];        // whole-tile counts
+  __shared__ int before[SCENE_INLINE_MAX];     // counts of the segments before this one
+  __shared__ int start[SCENE_INLINE_MAX + 1];
+  __shared__ int running[2][SCENE_INLINE_MAX];
+  __shared__ int wcnt[2][NW][SCENE_INLINE_MAX];
   const int* __restrict__ qk = pb.q_key + (size_t)ts * pb.R;
   const int* __restrict__ ql = pb.q_live + (size_t)ts * pb.R;
   int* __restrict__ qs = pb.q_shade + (size_t)ts * pb.QS;
@@ -233,7 +240,7 @@ __global__ void __launch_bounds__(BIN_T) k_bin_scatter(const PassBufs pb, const 
     const int used = (n + SEG_SLOTS - 1) / SEG_SLOTS;
     int tot = 0, bef = 0;
     for (int sg = 0; sg < used; ++sg) {
-      const int c = pb.seg_cnt[((size_t)ts * nseg + sg) * RAYN_MAX_HITABLES + tid];
+      const int c = pb.seg_cnt[((size_t)ts * nseg + sg) * SCENE_INLINE_MAX + tid];
       if (sg < seg) bef += c;
       tot += c;
     }
@@ -251,7 +258,7 @@ __global__ void __launch_bounds__(BIN_T) k_bin_scatter(const PassBufs pb, const 
     if (seg == 0) pb.n_slots[ts] = off;
   }
   __syncthreads();
-  if (seg == 0 && tid <= n_hit) pb.bin_start[ts * (RAYN_MAX_HITABLES + 1) + tid] = start[tid];
+  if (seg == 0 && tid <= n_hit) pb.bin_start[ts * (SCENE_INLINE_MAX + 1) + tid] = start[tid];
   // stable scatter of this segment, ONE barrier per 1024-ray chunk (double-buffered warp counts and bin cursors)
   int buf = 0;
   for (int base = lo; base < hi; base += BIN_T, buf ^= 1) {
@@ -278,6 +285,92 @@ __global__ void __launch_bounds__(BIN_T) k_bin_scatter(const PassBufs pb, const 
   }
   if (seg == 0 && tid < n_hit)
     for (int k = start[tid] + cnt[tid]; k < start[tid + 1]; ++k) qs[k] = -1;  // Ray::new_invalid padding
+}
+// The same partition for scenes of up to RAYN_MAX_HITABLES keys (after k_bin_count<RAYN_MAX_HITABLES>).  k_bin_scatter's one
+// ballot per key and chunk, and its [2][32][keys] warp counts (256 KB at 1024 keys), do not scale; here a warp ranks its rays
+// with __match_any_sync (rank among the warp's rays of the same key), the leader of each key group posts the group's size
+// in wcnt[warp][key], and a ray's slot is its bin cursor + the sizes posted by the warps before it + its rank.  A smaller
+// CTA keeps wcnt at 8 x 4 KB; the leaders clear their entries after use, so no chunk pays for the keys it does not touch.
+// Same order as k_bin_scatter: segments in order, chunks in order, warps in order, lanes in order.
+#define BINB_T 256
+__global__ void __launch_bounds__(BINB_T) k_bin_scatter_tables(const PassBufs pb, const int n_hit, const int nseg) {
+  constexpr int K = RAYN_MAX_HITABLES, NW = BINB_T / 32, PER = K / BINB_T;
+  static_assert(K % BINB_T == 0, "keys per thread of the bin scan");
+  const int seg = blockIdx.x, ts = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const unsigned lt = (1u << lane) - 1u;
+  const int n = pb.n_live[ts];
+  const int lo = seg * SEG_SLOTS, hi = min(n, lo + SEG_SLOTS);
+  if (lo >= n && seg > 0) return;
+  __shared__ int cnt[K];        // whole-tile counts
+  __shared__ int start[K + 1];  // bin starts (padded to x4)
+  __shared__ int running[K];    // write cursor of every bin in this segment
+  __shared__ int wcnt[NW][K];   // per-warp key counts of the current chunk, 0 where a warp has no such key
+  __shared__ int wsum[NW];
+  const int* __restrict__ qk = pb.q_key + (size_t)ts * pb.R;
+  const int* __restrict__ ql = pb.q_live + (size_t)ts * pb.R;
+  int* __restrict__ qs = pb.q_shade + (size_t)ts * pb.QS;
+  const int used = (n + SEG_SLOTS - 1) / SEG_SLOTS;
+  for (int k = tid; k < K; k += BINB_T) {
+    int tot = 0, bef = 0;
+    if (k < n_hit)
+      for (int sg = 0; sg < used; ++sg) {
+        const int c = pb.seg_cnt[((size_t)ts * nseg + sg) * K + k];
+        if (sg < seg) bef += c;
+        tot += c;
+      }
+    cnt[k] = tot, running[k] = bef;
+#pragma unroll
+    for (int w = 0; w < NW; ++w) wcnt[w][k] = 0;
+  }
+  __syncthreads();
+  // exclusive scan of the padded bin sizes (hitable.rs:100-111): thread t owns keys PER*t .. PER*t + PER-1
+  int sz[PER], s = 0;
+#pragma unroll
+  for (int q = 0; q < PER; ++q) s += (sz[q] = (cnt[PER * tid + q] + 3) & ~3);
+  int x = s;
+  for (int o = 1; o < 32; o <<= 1) {
+    const int y = __shfl_up_sync(0xffffffffu, x, o);
+    if (lane >= o) x += y;
+  }
+  if (lane == 31) wsum[warp] = x;
+  __syncthreads();
+  int off = x - s;
+  for (int w = 0; w < warp; ++w) off += wsum[w];
+#pragma unroll
+  for (int q = 0; q < PER; ++q) {
+    start[PER * tid + q] = off;
+    running[PER * tid + q] += off;
+    off += sz[q];
+  }
+  if (tid == BINB_T - 1) start[K] = off;
+  __syncthreads();
+  if (seg == 0) {
+    if (tid == 0) pb.n_slots[ts] = start[K];  // keys >= n_hit are empty: start[n_hit] == start[K]
+    for (int k = tid; k <= n_hit; k += BINB_T) pb.bin_start[(size_t)ts * (K + 1) + k] = start[k];
+  }
+  for (int base = lo; base < hi; base += BINB_T) {
+    const int i = base + tid;
+    const int id = i < hi ? ql[i] : -1;
+    const int key = i < hi ? qk[id] : -1;
+    const unsigned m = __match_any_sync(0xffffffffu, key);
+    const bool leader = key >= 0 && (m & lt) == 0;
+    if (leader) wcnt[warp][key] = __popc(m);
+    __syncthreads();
+    if (key >= 0) {
+      int o = running[key] + __popc(m & lt);
+      for (int w = 0; w < warp; ++w) o += wcnt[w][key];
+      qs[o] = id;
+    }
+    __syncthreads();
+    if (leader) {
+      atomicAdd(&running[key], __popc(m));  // read again only after the next chunk's first barrier
+      wcnt[warp][key] = 0;
+    }
+    __syncwarp();  // the clear above is ordered before this warp's posts of the next chunk
+  }
+  if (seg == 0)
+    for (int k = tid; k < n_hit; k += BINB_T)
+      for (int j = start[k] + cnt[k]; j < start[k + 1]; ++j) qs[j] = -1;  // Ray::new_invalid padding
 }
 
 // ---- pass-wide work distribution for the persistent march kernels: the per-tile live lists are
@@ -329,7 +422,8 @@ __global__ void __launch_bounds__(SCAN_T) k_scan_live(const PassBufs pb, int* __
 // a path is alive - 787 k empty blocks each, 5 % of a config-3 frame.  k_scan_slots (one CTA, after k_bin_scatter) lays the
 // NON-EMPTY 128-slot blocks of all tiles end to end; the kernels run a resident grid that strides over that list.
 #define SLOT_BLOCK 128
-__global__ void __launch_bounds__(SCAN_T) k_scan_slots(const __grid_constant__ DevScene sc, const PassBufs pb) {
+template <class Scn>
+__global__ void __launch_bounds__(SCAN_T) k_scan_slots(const __grid_constant__ Scn sc, const PassBufs pb) {
   __shared__ int wsum[SCAN_T / 32];
   __shared__ int carry;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -342,7 +436,7 @@ __global__ void __launch_bounds__(SCAN_T) k_scan_slots(const __grid_constant__ D
       const int i = base + tid;
       int v = 0;
       if (i < pb.n_tiles) {
-        const int* __restrict__ bs = pb.bin_start + i * (RAYN_MAX_HITABLES + 1);
+        const int* __restrict__ bs = pb.bin_start + i * (Scn::kMaxHit + 1);
         const int slots = row ? bs[hk + 1] - bs[hk] : pb.n_slots[i];
         v = (slots + SLOT_BLOCK - 1) / SLOT_BLOCK;
       }
@@ -372,6 +466,7 @@ __global__ void __launch_bounds__(SCAN_T) k_scan_slots(const __grid_constant__ D
     __syncthreads();
   }
 }
+template __global__ void k_scan_slots<DevScene>(const __grid_constant__ DevScene, const PassBufs);
 // The resident CTAs of a work-list kernel pull WORK_CHUNK consecutive 128-slot blocks at a time from a global counter (zeroed
 // by k_scan_live at the start of the depth).  Static striding was measured first: blocks differ 15x in cost (sky vs lit), the
 // slowest CTA ran ~10 % over the mean and k_shade_pre lost more than the empty blocks had cost.
@@ -419,7 +514,8 @@ RT_D int find_tile(const int* __restrict__ prefix, int n_tiles, int wb) {
 // persistent loop and cost more issue slots than the marches of cheap (sky) rays.  v4 keeps the
 // fold order of hitable.rs:177-198 but runs every maximal run of analytic spheres as a coherent
 // one-thread-per-ray kernel and every SDF hitable as a pure persistent march kernel.
-__global__ void __launch_bounds__(EXT_BATCH) k_extend_spheres(const __grid_constant__ DevScene sc, const PassBufs pb, const int first, const int last,
+template <class Scn>
+__global__ void __launch_bounds__(EXT_BATCH) k_extend_spheres(const __grid_constant__ Scn sc, const PassBufs pb, const int first, const int last,
                                                               const int init, const int moving, const int* __restrict__ batch_prefix,
                                                               int* __restrict__ work_ctr) {
   // the 128-ray batches of k_scan_live: no block is launched for rays that are gone
@@ -448,6 +544,7 @@ __global__ void __launch_bounds__(EXT_BATCH) k_extend_spheres(const __grid_const
     }
   })
 }
+template __global__ void k_extend_spheres<DevScene>(const __grid_constant__ DevScene, const PassBufs, const int, const int, const int, const int, const int*, int*);
 
 // ------------------------------------------------------------------------------------------
 // K2 sphere-march: TracedSDF::hit (sdf.rs:59-83, SURVEY §9.1) for SDF hitable `hk` over every live
@@ -482,8 +579,8 @@ __global__ void __launch_bounds__(EXT_BATCH) k_extend_spheres(const __grid_const
 #define RAYN_MARCH_OCC_BULB RAYN_MARCH_OCC  // same for the authored Mandelbulb estimator (needs more registers; tuning hook)
 #endif
 #define MARCH_OCC(V) ((V) == SDFV_BULB ? RAYN_MARCH_OCC_BULB : RAYN_MARCH_OCC)
-template <int V>
-__global__ void __launch_bounds__(EXT_T, MARCH_OCC(V)) k_extend_march(const __grid_constant__ DevScene sc, const PassBufs pb, const Thr thr,
+template <int V, class Scn>
+__global__ void __launch_bounds__(EXT_T, MARCH_OCC(V)) k_extend_march(const __grid_constant__ Scn sc, const PassBufs pb, const Thr thr,
                                                           const int hk, const int spheres_first, const int* __restrict__ batch_prefix,
                                                           int* __restrict__ work_ctr) {
   const SdfK k = make_sdfk(sc.hit[hk], sc.one);  // fractal constants: kernel-parameter bank -> registers, once
@@ -615,14 +712,14 @@ __global__ void __launch_bounds__(EXT_T, MARCH_OCC(V)) k_extend_march(const __gr
 // sdfu's tetrahedral normals_fast (oracle/README.md A8) = 4 distance evaluations = 2 packed evaluations
 // per lane, specialised on the SDF like the march kernels.  Writes nrm[g] = (normal, offset_by).
 // ------------------------------------------------------------------------------------------
-template <int V>
-__global__ void __launch_bounds__(128, 8) k_normals(const __grid_constant__ DevScene sc, const PassBufs pb, const Thr thr, const int hk, const int j,
+template <int V, class Scn>
+__global__ void __launch_bounds__(128, 8) k_normals(const __grid_constant__ Scn sc, const PassBufs pb, const Thr thr, const int hk, const int j,
                                                     int* __restrict__ work_ctr) {
   const int* __restrict__ prefix = pb.slot_prefix + (size_t)(1 + j) * pb.prefix_stride;  // 128-slot blocks of this SDF's bins, all tiles
   const SdfK k = make_sdfk(sc.hit[hk], sc.one);
   int evals = 0;
   FOR_EACH_WORK_BLOCK(prefix, pb.n_tiles, work_ctr, {
-    const int* __restrict__ bs = pb.bin_start + ts * (RAYN_MAX_HITABLES + 1);
+    const int* __restrict__ bs = pb.bin_start + ts * (Scn::kMaxHit + 1);
     const int s = bs[hk] + local * SLOT_BLOCK + threadIdx.x;
     const int id = s < bs[hk + 1] ? pb.q_shade[(size_t)ts * pb.QS + s] : -1;
     if (id >= 0) {  // < 0: beyond the bin, or a padding lane (hitable.rs:100-111)
@@ -701,7 +798,8 @@ struct SlotCtx {  // what pre and post both derive for a shading slot
 // utilisation): everything a slot needs hangs off ONE dependent load, its path id, so that the hit object (q_key is indexed
 // by path), the pixel's scramble value and the sampler-table entries are all in flight together - the former search of the
 // tile's bin_start row was a chain of up to n_hit dependent loads.
-RT_D SlotCtx slot_ctx(const DevScene& sc, const DevFrame& fr, const PassBufs& pb, int ts, int s, int nslots, int depth, int lane) {
+template <class Scn>
+RT_D SlotCtx slot_ctx(const Scn& sc, const DevFrame& fr, const PassBufs& pb, int ts, int s, int nslots, int depth, int lane) {
   SlotCtx c;
   const int* __restrict__ qs = pb.q_shade + (size_t)ts * pb.QS;
   c.id = s < nslots ? qs[s] : -1;
@@ -738,7 +836,8 @@ RT_D SlotCtx slot_ctx(const DevScene& sc, const DevFrame& fr, const PassBufs& pb
   return c;
 }
 
-RT_D void shade_pre_slot(const DevScene& sc, const DevFrame& fr, const PassBufs& pb, const int depth, const Thr thr, const int ts, const int s) {
+template <class Scn>
+RT_D void shade_pre_slot(const Scn& sc, const DevFrame& fr, const PassBufs& pb, const int depth, const Thr thr, const int ts, const int s) {
   const int nslots = pb.n_slots[ts];
   if ((s & ~31) >= nslots) return;  // warp-uniform
   const SlotCtx cx = slot_ctx(sc, fr, pb, ts, s, nslots, depth, threadIdx.x & 31);
@@ -837,11 +936,13 @@ RT_D void shade_pre_slot(const DevScene& sc, const DevFrame& fr, const PassBufs&
 #ifndef RAYN_SHADE_PRE_OCC
 #define RAYN_SHADE_PRE_OCC 8  // resident CTAs per SM k_shade_pre is compiled for (tuning hook)
 #endif
-__global__ void __launch_bounds__(128, RAYN_SHADE_PRE_OCC) k_shade_pre(const __grid_constant__ DevScene sc, const DevFrame fr, const PassBufs pb,
+template <class Scn>
+__global__ void __launch_bounds__(128, RAYN_SHADE_PRE_OCC) k_shade_pre(const __grid_constant__ Scn sc, const DevFrame fr, const PassBufs pb,
                                                       const int depth, const Thr thr, int* __restrict__ work_ctr) {
   // row 0 of the work lists: the non-empty 128-slot blocks of every tile's shading queue
   FOR_EACH_WORK_BLOCK(pb.slot_prefix, pb.n_tiles, work_ctr, { shade_pre_slot(sc, fr, pb, depth, thr, ts, local * SLOT_BLOCK + threadIdx.x); })
 }
+template __global__ void k_shade_pre<DevScene>(const __grid_constant__ DevScene, const DevFrame, const PassBufs, const int, const Thr, int*);
 
 // ------------------------------------------------------------------------------------------
 // K5 shadow sphere-march: TracedSDF::occluded per slot (sdf.rs:25-57, SURVEY §9.2) over the segment
@@ -851,8 +952,8 @@ __global__ void __launch_bounds__(128, RAYN_SHADE_PRE_OCC) k_shade_pre(const __g
 // ------------------------------------------------------------------------------------------
 #define SHD_T 128
 #define SHD_BATCH 128
-template <int V>
-__global__ void __launch_bounds__(SHD_T, MARCH_OCC(V)) k_shadow(const __grid_constant__ DevScene sc, const PassBufs pb, const int hk, const int j,
+template <int V, class Scn>
+__global__ void __launch_bounds__(SHD_T, MARCH_OCC(V)) k_shadow(const __grid_constant__ Scn sc, const PassBufs pb, const int hk, const int j,
                                                     int* __restrict__ work_ctr) {
   const SdfK k = make_sdfk(sc.hit[hk], sc.one);
   const int lane = threadIdx.x & 31;
@@ -958,7 +1059,8 @@ __global__ void __launch_bounds__(SHD_T, MARCH_OCC(V)) k_shadow(const __grid_con
   if (V == SDFV_BULB) warp_add(pb.counters + CNT_BULB_ITERS_SHADOW, bulb_iters);
 }
 
-RT_D void shade_post_slot(const DevScene& sc, const DevFrame& fr, const PassBufs& pb, const int depth, const int pre_n, const int ts, const int s) {
+template <class Scn>
+RT_D void shade_post_slot(const Scn& sc, const DevFrame& fr, const PassBufs& pb, const int depth, const int pre_n, const int ts, const int s) {
   const int nslots = pb.n_slots[ts];
   if ((s & ~31) >= nslots) return;
   const SlotCtx cx = slot_ctx(sc, fr, pb, ts, s, nslots, depth, threadIdx.x & 31);
@@ -1043,10 +1145,12 @@ RT_D void shade_post_slot(const DevScene& sc, const DevFrame& fr, const PassBufs
   }
 }
 
-__global__ void __launch_bounds__(128, 8) k_shade_post(const __grid_constant__ DevScene sc, const DevFrame fr, const PassBufs pb,
+template <class Scn>
+__global__ void __launch_bounds__(128, 8) k_shade_post(const __grid_constant__ Scn sc, const DevFrame fr, const PassBufs pb,
                                                        const int depth, const int pre_n, int* __restrict__ work_ctr) {
   FOR_EACH_WORK_BLOCK(pb.slot_prefix, pb.n_tiles, work_ctr, { shade_post_slot(sc, fr, pb, depth, pre_n, ts, local * SLOT_BLOCK + threadIdx.x); })
 }
+template __global__ void k_shade_post<DevScene>(const __grid_constant__ DevScene, const DevFrame, const PassBufs, const int, const int, int*);
 
 // ------------------------------------------------------------------------------------------
 // K6 compact: film.rs:604-625.  Order-preserving stream compaction of the surviving slots of
@@ -1070,7 +1174,7 @@ __global__ void __launch_bounds__(CMP_T) k_compact_count(const PassBufs pb, cons
   __syncthreads();
   if ((tid & 31) == 0 && c) atomicAdd(&tot, c);
   __syncthreads();
-  if (tid == 0) pb.seg_cnt[((size_t)ts * nseg + seg) * RAYN_MAX_HITABLES] = tot;
+  if (tid == 0) pb.seg_cnt[((size_t)ts * nseg + seg) * SCENE_INLINE_MAX] = tot;
 }
 __global__ void __launch_bounds__(CMP_T) k_compact_scatter(const PassBufs pb, const int nseg) {
   const int seg = blockIdx.x, ts = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1086,7 +1190,7 @@ __global__ void __launch_bounds__(CMP_T) k_compact_scatter(const PassBufs pb, co
     const int used = (n + SEG_SLOTS - 1) / SEG_SLOTS;
     int bef = 0, tot = 0;
     for (int sg = 0; sg < used; ++sg) {
-      const int c = pb.seg_cnt[((size_t)ts * nseg + sg) * RAYN_MAX_HITABLES];
+      const int c = pb.seg_cnt[((size_t)ts * nseg + sg) * SCENE_INLINE_MAX];
       if (sg < seg) bef += c;
       tot += c;
     }
@@ -1546,7 +1650,8 @@ __global__ void k_kat_sdf_hit(const RaynHitable h, const RaynRenderConsts rc, lo
   out[i] = sdf_hit(h, rc, mk3(o3[3 * i], o3[3 * i + 1], o3[3 * i + 2]), mk3(d3[3 * i], d3[3 * i + 1], d3[3 * i + 2]), t_max[i],
                    thr, &ev);
 }
-__global__ void k_kat_occluded(const __grid_constant__ DevScene sc, long long n, const float* s3, const float* e3, float* out) {
+template <class Scn>
+__global__ void k_kat_occluded(const __grid_constant__ Scn sc, long long n, const float* s3, const float* e3, float* out) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   int ev = 0;
@@ -1559,7 +1664,9 @@ __global__ void k_kat_occluded(const __grid_constant__ DevScene sc, long long n,
   const float fast = test_occluded(sc, a, b, &ev);
   out[i] = acc == fast ? acc : -1.0f;  // -1 flags a disagreement between the two forms
 }
-__global__ void k_kat_closest_hit(const __grid_constant__ DevScene sc, Thr thr, long long n, const float* o3, const float* d3,
+template __global__ void k_kat_occluded<DevScene>(const __grid_constant__ DevScene, long long, const float*, const float*, float*);
+template <class Scn>
+__global__ void k_kat_closest_hit(const __grid_constant__ Scn sc, Thr thr, long long n, const float* o3, const float* d3,
                                   float* out_t, int* out_obj) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -1567,6 +1674,7 @@ __global__ void k_kat_closest_hit(const __grid_constant__ DevScene sc, Thr thr, 
   closest_hit(sc, mk3(o3[3 * i], o3[3 * i + 1], o3[3 * i + 2]), mk3(d3[3 * i], d3[3 * i + 1], d3[3 * i + 2]), thr, &out_t[i],
               &out_obj[i], &ev);
 }
+template __global__ void k_kat_closest_hit<DevScene>(const __grid_constant__ DevScene, Thr, long long, const float*, const float*, float*, int*);
 
 __global__ void k_kat_light_sample(const RaynLight L, long long n, const float* s0, const float* s1, const float* p3, float* out_pt3, float* out_pdf) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;

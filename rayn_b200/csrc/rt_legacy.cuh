@@ -78,7 +78,7 @@ __global__ void __launch_bounds__(128) k_shade(const __grid_constant__ DevScene 
   int evals = 0, shadows = 0;
   if (valid) {
     // object of this slot from the tile's bin table
-    const int* __restrict__ bs = pb.bin_start + ts * (RAYN_MAX_HITABLES + 1);
+    const int* __restrict__ bs = pb.bin_start + ts * (SCENE_INLINE_MAX + 1);
     int obj = 0;
     while (obj + 1 < sc.n_hit && s >= bs[obj + 1]) ++obj;
     const RaynHitable& h = sc.hit[obj];
